@@ -3,6 +3,7 @@
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference]
                     [--config cfg2|cfg3|cfg4|cfg5|cfg5stress] [--scaling weak|strong] [--batch B]
+                    [--dump-outputs DIR]
     (N > 1: python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...)
 
 Workloads (BASELINE.json configs[1..4], SURVEY 8d; synthetic uint8 images seed 1234, synthetic weights with the
@@ -34,6 +35,9 @@ stack of step i+1; every step's work is inside the timed region (the region ends
             create_model / Decoder / extract_targets / MultiBoxLoss on this host's cores, on a bounded sample of
             the same workload (kind "reference"); the oracle port (kind "port") only if oracle/_ref is absent.
 --impl reference times that CPU path alone and never imports ssds_pytorch_b200.
+--dump-outputs DIR  after the timed steps, rank 0 writes what the last device-resident step returned as DIR/<name>.npy
+            (detect: scores [B,100], boxes [B,100,4], classes [B,100]; cfg4: loss [3] = cls_loss, loc_loss,
+            fg_targets), float32, so that two builds can be compared output for output on the same seeded inputs.
 """
 import argparse
 import json
@@ -42,6 +46,8 @@ import subprocess
 import sys
 import threading
 import time
+
+import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
@@ -251,7 +257,7 @@ def run_reference(args):
         return
     c = CONFIGS[args.config]
     n = args.cpu_images or c["cpu_images"]
-    steps = max(1, min(args.steps, 3))
+    steps = args.steps
     sec, base = cpu_baseline(args.config, n, steps)
     v = n / sec
     line = {"impl": "reference", "metric": METRIC, "value": v, "unit": "images/s", "n_gpus": args.gpus,
@@ -300,6 +306,22 @@ def _self_check(name, sd, dev_in, plan_outputs, make_model):
     torch.cuda.empty_cache()
     return ("timed plan (multi-way/resident/paired/fused-block launches, CUDA-graph replay) == 1-way unpaired "
             "un-fused eager plan, bit for bit")
+
+
+DUMP_LIMIT = 64 << 20
+
+
+def dump_outputs(outdir, arrays):
+    """One float32 .npy per output; above DUMP_LIMIT bytes in all, a fixed seeded sample of the images."""
+    arrays = {k: np.asarray(v, np.float32) for k, v in arrays.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_LIMIT:
+        B = next(iter(arrays.values())).shape[0]
+        keep = np.sort(np.random.default_rng(0).choice(B, max(1, B * DUMP_LIMIT // total), replace=False))
+        arrays = {k: v[keep] for k, v in arrays.items()}
+    os.makedirs(outdir, exist_ok=True)
+    for k, v in arrays.items():
+        np.save(os.path.join(outdir, k + ".npy"), v)
 
 
 def run_b200(args):
@@ -357,12 +379,13 @@ def run_b200(args):
         def step_device():
             # decode + NMS (+ all-gather) of this step run on the detector's side stream and overlap the
             # conv stack of the next step; det.join() below makes the timed region wait for them
-            det.detect_device(dev_in, overlap=True, packed_out=packed)
+            out = det.detect_device(dev_in, overlap=True, packed_out=packed)
             if world > 1:
                 with torch.cuda.stream(det._post_stream):
                     gather_detections(packed)
                     det._post_done = torch.cuda.Event()
                     det._post_done.record(det._post_stream)
+            return out
 
         def step_host(i):
             return det.detect_host(host[i % 2], slot=i % 2, gather=world > 1)
@@ -380,7 +403,7 @@ def run_b200(args):
             return LossStep(cfg_dict(name), sd, device=device, use_graph=False).model
 
         def step_device():
-            ls.loss_device(dev_in, tg_dev)
+            return ls.loss_device(dev_in, tg_dev)
 
         def step_host(i):
             return ls.loss_host(host[i % 2], tg_host)
@@ -429,12 +452,17 @@ def run_b200(args):
     sampler.active = True
     e0.record()
     for _ in range(K):
-        step_device()
+        last = step_device()
     join()
     e1.record()
     barrier()
     sampler.active = False
     dev_ms = e0.elapsed_time(e1)
+    if args.dump_outputs and rank == 0:
+        names = ["scores", "boxes", "classes"] if detect else ["loss"]
+        last = last if detect else (last,)
+        dumped = {n: t.float().cpu().numpy() for n, t in zip(names, last)}
+    del last
 
     # ---- e2e: pinned host batch -> H2D -> step -> D2H, every step ----
     barrier()
@@ -540,6 +568,8 @@ def run_b200(args):
         if world == 1 and not args.no_cpu:
             _, line["cpu_baseline"] = cpu_baseline(name, args.cpu_images or c["cpu_images"], 1)
         print(json.dumps(line))
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, dumped)
     if world > 1:
         dist.destroy_process_group()
 
@@ -557,7 +587,13 @@ def main():
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-selfcheck", action="store_true")
     ap.add_argument("--no-sections", action="store_true", help="skip the per-group roofline timings")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the last timed step's outputs as DIR/<name>.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the B200 path (--impl b200)")
     if args.impl == "reference":
         run_reference(args)
     else:

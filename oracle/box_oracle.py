@@ -246,6 +246,51 @@ def decoder_call(loc, conf, anchors, conf_threshold, nms_threshold, top_n, top_n
     return nms(*decoded, nms=nms_threshold, ndetections=top_n, using_diou=use_diou)
 
 
+def mean_average_precision(detections, targets, num_classes, conf_threshold, iou_threshold):
+    """reference evaluation_metrics.py:5-142 — ``detections`` = (scores [B,D], boxes [B,D,4], classes [B,D]),
+    ``targets`` = per image [T,5] (x1, y1, x2, y2, class).  Per image and class, each detection above
+    conf_threshold takes the target it overlaps most and is a true positive if that IoU reaches iou_threshold and
+    the target is still free.  AP per class is the area under the precision/recall curve with precision made
+    non-increasing (VOC all-point); classes without targets are NaN and left out of the mean."""
+    hits = [([], []) for _ in range(num_classes)]
+    npos = np.zeros(num_classes, np.int64)
+    for s, b, c, t in zip(*(np.asarray(a) for a in detections), targets):
+        t = np.asarray(t, np.float32)
+        keep = s > conf_threshold
+        s, b, c = s[keep], b[keep].astype(np.float32), c[keep]
+        for k in range(num_classes):
+            tk, sk, bk = t[t[:, 4] == k, :4], s[c == k], b[c == k]
+            npos[k] += len(tk)
+            tp = np.zeros(len(sk), bool)
+            if len(sk) and len(tk):
+                lt = np.maximum(bk[:, None, :2], tk[:, :2])
+                rb = np.minimum(bk[:, None, 2:], tk[:, 2:])
+                inter = np.prod(rb - lt, axis=2) * (lt < rb).all(axis=2)
+                area_b = np.prod(bk[:, 2:] - bk[:, :2], axis=1)
+                area_t = np.prod(tk[:, 2:] - tk[:, :2], axis=1)
+                iou = inter / (area_b[:, None] + area_t - inter)
+                taken = np.zeros(len(tk), bool)
+                for i, j in enumerate(iou.argmax(axis=1)):
+                    if iou[i, j] >= iou_threshold and not taken[j]:
+                        taken[j] = tp[i] = True
+            hits[k][0].extend(sk.tolist())
+            hits[k][1].extend(tp.tolist())
+    aps = []
+    for k in range(num_classes):
+        if npos[k] == 0:
+            aps.append(np.nan)
+            continue
+        order = np.argsort(np.asarray(hits[k][0], np.float64))[::-1]
+        tp = np.asarray(hits[k][1], np.int64)[order]
+        ctp, cfp = np.cumsum(tp), np.cumsum(1 - tp)
+        rec = np.concatenate([[0], ctp / float(npos[k]), [1]])
+        prec = np.concatenate([[0], ctp / np.maximum(ctp + cfp, np.finfo(np.float64).eps), [0]])
+        prec = np.maximum.accumulate(prec[::-1])[::-1]
+        step = np.nonzero(rec[1:] != rec[:-1])[0] + 1
+        aps.append(np.sum((rec[step] - rec[step - 1]) * prec[step]))
+    return float(np.nanmean(aps))
+
+
 # --------------------------------------------------------------------------- #
 # match ("jaccard" + "match" + "encode")
 # --------------------------------------------------------------------------- #

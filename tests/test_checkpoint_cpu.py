@@ -1,12 +1,13 @@
 """Weight import (SURVEY 8f rank 2): ssds_pytorch_b200.checkpoint against the reference's own
-ssds/core/checkpoint.py — checkpoints WRITTEN by the reference's `save_checkpoints`, read back by both the
-reference's `resume_checkpoint` (into a fresh reference model) and our `load_checkpoint`, results compared
-tensor by tensor.  Needs /root/reference (authoring container); the self-contained cases below it do not.
+ssds/core/checkpoint.py — a checkpoint laid out as the reference's `save_checkpoints` writes it, read back by our
+`find_previous_checkpoint` / `load_checkpoint` and compared key by key with what the reference's
+`resume_checkpoint` made of the same file (tests/golden/reference_state_dicts.json.gz, written by
+tests/golden/make_golden_reference.py).
 """
+import gzip
+import json
 import os
-import sys
-import warnings
-from collections import OrderedDict, defaultdict
+from collections import OrderedDict
 
 import pytest
 import torch
@@ -14,10 +15,14 @@ import torch
 from ssds_pytorch_b200 import checkpoint as CK
 from ssds_pytorch_b200 import synth
 
-REF = os.environ.get("SSDS_REFERENCE", "/root/reference")
+GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "reference_state_dicts.json.gz")
 FL = [[3, 4, 5, "Conv:S"], [128, 256, 512, 256]]
 CFG = {"MODEL": {"SSDS": "SSD", "NETS": "ResNet18", "IMAGE_SIZE": [96, 160], "NUM_CLASSES": 20, "FEATURE_LAYER": FL,
                  "SIZES": [[2.0, 2.828]] * 4, "ASPECT_RATIOS": [[1, 2, 0.5]] * 4}}
+# the reference round trip: weights of seed CKPT_SEED saved from a DataParallel model (`module.` keys) as
+# <prefix>_epoch_<epoch>.pth, resumed into a model holding the weights of seed BASE_SEED under each scope
+CKPT_SEED, BASE_SEED, CKPT_PREFIX, CKPT_EPOCH = 0, 1, "ssd_resnet18_x", 3
+SCOPES = ("", "backbone,extras")
 
 
 def _sd(seed):
@@ -65,42 +70,29 @@ def _write_cfg(tmp_path):
     return p
 
 
-@pytest.mark.skipif(not os.path.isdir(os.path.join(REF, "ssds")), reason="needs the reference tree")
-def test_against_reference_save_and_resume(tmp_path, capsys):
-    sys.path.insert(0, REF)
-    warnings.filterwarnings("ignore")
-    import torchvision as tv
-    tv.models.resnet.model_urls = defaultdict(lambda: None)        # no download (SURVEY 8c)
-    tv.models.densenet.model_urls = defaultdict(lambda: None)
-    tv.models.mobilenet.model_urls = defaultdict(lambda: None)
-    try:
-        from ssds.core import checkpoint as RCK
-        from ssds.core import config as rcfg
-        from ssds.modeling import model_builder
-    except Exception as e:                                         # reference imports that this image lacks
-        pytest.skip(f"reference not importable here: {e}")
-    m = rcfg.cfg.MODEL
-    m.SSDS, m.NETS, m.IMAGE_SIZE, m.NUM_CLASSES = "SSD", "ResNet18", [96, 160], 20
-    m.FEATURE_LAYER, m.SIZES, m.ASPECT_RATIOS = FL, CFG["MODEL"]["SIZES"], CFG["MODEL"]["ASPECT_RATIOS"]
-    torch.manual_seed(0)
-    trained = model_builder.create_model(m)
-    with torch.no_grad():
-        for p in trained.parameters():
-            p.add_(torch.randn_like(p) * 0.01)
-    RCK.save_checkpoints(torch.nn.DataParallel(trained), str(tmp_path), "ssd_resnet18_x", 3)     # `module.` keys
-    epochs, files = CK.find_previous_checkpoint(str(tmp_path))
-    assert (epochs, files) == RCK.find_previous_checkpoint(str(tmp_path))
-    for scope in ("", "backbone,extras"):
-        torch.manual_seed(1)
-        fresh = model_builder.create_model(m)
-        base = OrderedDict((k, v.clone()) for k, v in fresh.state_dict().items())
-        RCK.resume_checkpoint(fresh, files[-1], scope)
-        got, rep = CK.load_checkpoint(files[-1], scope, base)
-        ref = fresh.state_dict()
-        assert list(got) == list(ref)
-        for k in ref:
-            assert torch.equal(got[k], ref[k]), (scope, k)
+def test_against_reference_save_and_resume(tmp_path):
+    with gzip.open(GOLDEN, "rt") as f:
+        ref = json.load(f)["checkpoint"]
+    d = str(tmp_path)
+    saved = _sd(CKPT_SEED)
+    assert sorted(ref["saved_keys"]) == sorted("module." + k for k in saved)
+    torch.save(OrderedDict((k, saved[k[len("module."):]]) for k in ref["saved_keys"]),
+               os.path.join(d, f"{CKPT_PREFIX}_epoch_{CKPT_EPOCH}.pth"))
+    with open(os.path.join(d, "checkpoint_list.txt"), "w") as f:
+        f.write(ref["index"].replace("{dir}", d))
+    epochs, files = CK.find_previous_checkpoint(d)
+    assert [epochs, files] == [ref["found"][0], [p.replace("{dir}", d) for p in ref["found"][1]]]
+    for scope in SCOPES:
+        want = ref["scopes"][scope]
+        base = _sd(BASE_SEED)
+        got, rep = CK.load_checkpoint(files[-1], scope, OrderedDict((k, v.clone()) for k, v in base.items()))
+        assert list(got) == want["keys"]
+        for k in got:
+            src = want["source"][k]
+            if src in ("checkpoint", "both"):
+                assert torch.equal(got[k], saved[k]), (scope, k)
+            if src in ("base", "both"):
+                assert torch.equal(got[k], base[k]), (scope, k)
         assert CK.check_state_dict(CFG, got)["ok"]
         if scope:
             assert rep["unresumed"] and all("backbone" not in k and "extras" not in k for k in rep["unresumed"])
-    capsys.readouterr()

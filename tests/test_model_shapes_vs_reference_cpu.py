@@ -1,19 +1,15 @@
 """`synth.model_shapes` (the layer table checkpoint validation and the synthetic weights rely on) against the
-reference's own `create_model(cfg).state_dict()` for every engine combination model.ENGINES offers.
-Needs /root/reference (authoring container); skipped elsewhere."""
+reference's own `create_model(cfg).state_dict()` for every engine combination model.ENGINES offers, as stored in
+tests/golden/reference_state_dicts.json.gz by tests/golden/make_golden_reference.py."""
+import gzip
+import json
 import os
-import sys
-import warnings
-from collections import defaultdict
-from functools import partial
 
 import pytest
-import torch
 
 from ssds_pytorch_b200 import synth
 
-REF = os.environ.get("SSDS_REFERENCE", "/root/reference")
-pytestmark = pytest.mark.skipif(not os.path.isdir(os.path.join(REF, "ssds")), reason="needs the reference tree")
+GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "reference_state_dicts.json.gz")
 
 FPN = [[3, 4, 5, "Conv:S", "Conv:S"], [512, 1024, 2048, 2048, 256]]
 CASES = {
@@ -36,37 +32,15 @@ CASES = {
 
 @pytest.fixture(scope="module")
 def ref():
-    sys.path.insert(0, REF)
-    warnings.filterwarnings("ignore")
-    try:
-        import torchvision as tv
-        tv.models.resnet.model_urls = defaultdict(lambda: None)        # url=None: initialize() skips the download
-        tv.models.densenet.model_urls = defaultdict(lambda: None)
-        from torchvision.models import mobilenetv2 as mv2
-        tv.models.mobilenet.model_urls = defaultdict(lambda: None)
-        tv.models.mobilenet._make_divisible = mv2._make_divisible
-        tv.models.mobilenet.InvertedResidual = mv2.InvertedResidual
-        tv.models.mobilenet.ConvBNReLU = partial(tv.ops.misc.Conv2dNormActivation, norm_layer=torch.nn.BatchNorm2d,
-                                                 activation_layer=torch.nn.ReLU6)
-        from ssds.modeling.nets import regnet
-        regnet.RegNet.initialize = lambda self: None                   # hard-coded URLs, no network (SURVEY 8c)
-        from ssds.core import config as rcfg
-        from ssds.modeling import model_builder
-    except Exception as e:
-        pytest.skip(f"reference not importable here: {e}")
-    return rcfg, model_builder
+    with gzip.open(GOLDEN, "rt") as f:
+        return json.load(f)["state_dicts"]
 
 
 @pytest.mark.parametrize("name", list(CASES))
 def test_layer_table_equals_reference_state_dict(ref, name):
-    rcfg, model_builder = ref
     ssds, nets, fl = CASES[name]
     L = len(fl[0])
-    m = rcfg.cfg.MODEL
-    m.SSDS, m.NETS, m.IMAGE_SIZE, m.NUM_CLASSES = ssds, nets, [128, 128], 20
-    m.FEATURE_LAYER, m.SIZES, m.ASPECT_RATIOS = fl, [[2.0, 2.828]] * L, [[1, 2, 0.5]] * L
-    model = model_builder.create_model(m)
-    want = [(k, tuple(v.shape)) for k, v in model.state_dict().items()]
+    want = [(k, tuple(s)) for k, s in ref[name]]
     got = [(k, tuple(s)) for k, s in synth.model_shapes(ssds, nets, fl, [6] * L, 20)]
     assert [k for k, _ in got] == [k for k, _ in want]                 # same keys, same ORDER
     assert got == want

@@ -1,12 +1,15 @@
-"""tcgen05 implicit-GEMM convolution vs a torch fp32 reference of the same op on bf16-rounded
-operands (the kernel multiplies bf16 x bf16 exactly and accumulates in fp32, so the only
-differences are fp32 summation order and the final bf16 rounding of the output).
-Tolerance (written here, as the task requires): |err| <= 2e-2 * max(1, |ref|) for bf16 outputs
-(1 bf16 ulp = 0.4-0.8 %), 1e-3 for fp32 head outputs."""
+"""tcgen05 implicit-GEMM convolution vs an fp64 reference of the same op on the kernel's bf16 operands (the kernel
+multiplies bf16 x bf16 exactly and accumulates in fp32, so the only differences are fp32 summation order and the final
+bf16 rounding of the output).
+Tolerance: bf16 outputs within half a bf16 ulp plus the fp32 accumulation error (oracle/bf16_bound.py).  The stems
+keep |err| <= 2e-2 * max(1, |ref|): their reference normalises the image itself instead of consuming the bf16 tensor
+pack_image_s2d produces.  The fp32 head: loc within 2^-17 * S, the sigmoid-ed conf (computed with __expf) 1e-4."""
 import numpy as np
 import pytest
 import torch
 import torch.nn.functional as F
+
+from oracle.bf16_bound import ACC_REL, assert_bf16_close, conv_ref64
 
 pytestmark = pytest.mark.gpu
 
@@ -19,18 +22,6 @@ def K():
     torch.backends.cuda.matmul.allow_tf32 = False
     from ssds_pytorch_b200 import conv
     return conv
-
-
-def ref_conv(x_nhwc, w, b, stride, pad, relu, residual=None):
-    x = x_nhwc.float().permute(0, 3, 1, 2)
-    y = F.conv2d(x, w.to(torch.bfloat16).float(), b, stride=stride, padding=pad)
-    if residual is not None:
-        y = y + residual.float().permute(0, 3, 1, 2)
-    if relu:
-        y = y.relu()
-    if relu == 2:
-        y = y.clamp(max=6.0)
-    return y.permute(0, 2, 3, 1)
 
 
 CASES = [
@@ -66,10 +57,9 @@ def test_conv_nhwc(K, case):
     res = torch.randn((N, Ho, Wo, Cout), generator=g).to(torch.bfloat16).cuda() if use_res else None
     y = K.conv2d(x, K.pack_weight(w).cuda(), b.cuda(), k, k, stride, pad, relu, res)
     torch.cuda.synchronize()
-    ref = ref_conv(x, w.cuda(), b.cuda(), stride, pad, relu, res)
-    err = (y.float() - ref).abs() / ref.abs().clamp(min=1.0)
-    assert err.max().item() <= 2e-2, f"max rel err {err.max().item()}"
-    assert torch.isfinite(y.float()).all()
+    ref, S = conv_ref64(x, w, b, stride, pad, residual=res, relu=int(relu))
+    worst = assert_bf16_close(y, ref, S, str(case))
+    print(f"conv {case}: worst err/tol {worst:.3f}")
 
 
 def test_conv_head_split_sigmoid(K):
@@ -82,13 +72,18 @@ def test_conv_head_split_sigmoid(K):
     for sig in (True, False):
         loc, conf = K.conv2d_head(x, K.pack_weight(w).cuda(), b.cuda(), A * 4, sig)
         torch.cuda.synchronize()
-        ref = F.conv2d(x.float().permute(0, 3, 1, 2), w.to(torch.bfloat16).float().cuda(), b.cuda(), padding=1)
+        ref, S = conv_ref64(x, w, b, 1, 1)
+        ref, S = ref.permute(0, 3, 1, 2), S.permute(0, 3, 1, 2)
         rl, rc = ref[:, :A * 4], ref[:, A * 4:]
         if sig:
             rc = rc.sigmoid()
         assert loc.shape == rl.shape and conf.shape == rc.shape
-        assert (loc - rl).abs().max().item() <= 1e-3
-        assert (conf - rc).abs().max().item() <= (1e-4 if sig else 1e-3)
+        # fp32 outputs: fp32 accumulation error only (no bf16 rounding)
+        assert ((loc.double() - rl).abs() <= ACC_REL * S[:, :A * 4]).all(), ((loc.double() - rl).abs().max().item())
+        if sig:
+            assert (conf.double() - rc).abs().max().item() <= 1e-4
+        else:
+            assert ((conf.double() - rc).abs() <= ACC_REL * S[:, A * 4:]).all()
 
 
 def test_stem_s2d_equals_7x7s2(K):
@@ -149,15 +144,10 @@ def test_dwconv3x3(K, case):
     b = torch.randn((Cc,), generator=g) * 0.2
     y = K.dwconv3x3(x, K.pack_dw_weight(w).cuda(), b.cuda(), stride, relu)
     torch.cuda.synchronize()
-    ref = F.conv2d(x.float().permute(0, 3, 1, 2), w.to(torch.bfloat16).float().cuda(), b.cuda(), stride=stride,
-                   padding=1, groups=Cc)
-    if relu:
-        ref = ref.relu()
-    if relu == 2:
-        ref = ref.clamp(max=6.0)
-    ref = ref.permute(0, 2, 3, 1)
-    err = (y.float() - ref).abs() / ref.abs().clamp(min=1.0)
-    assert y.shape == ref.shape and err.max().item() <= 1e-2, err.max().item()
+    ref, S = conv_ref64(x, w, b, stride, 1, groups=Cc, relu=relu)
+    assert y.shape == ref.shape
+    worst = assert_bf16_close(y, ref, S, str(case))
+    print(f"dwconv3x3 {case}: worst err/tol {worst:.3f}")
 
 
 RAGGED = [
@@ -201,9 +191,9 @@ def test_conv_ragged_cout_staged_equals_direct(K, case, monkeypatch):
         outs.append(y.clone())
     monkeypatch.delenv("SSDSB_DIRECT_RAGGED", raising=False)
     assert torch.equal(outs[0], outs[1])
-    ref = ref_conv(x, w.cuda(), b, stride, pad, relu, res)
-    err = (outs[0].float() - ref).abs() / ref.abs().clamp(min=1.0)
-    assert err.max().item() <= 2e-2, err.max().item()
+    ref, S = conv_ref64(x, w, b, stride, pad, residual=res, relu=relu)
+    worst = assert_bf16_close(outs[0], ref, S, str(case))
+    print(f"ragged {case}: worst err/tol {worst:.3f}")
 
 
 @pytest.mark.parametrize("case", [(2, 75, 75, 160, 1, 2), (1, 150, 150, 96, 2, 2), (2, 19, 19, 384, 1, 2),
@@ -266,6 +256,9 @@ MBCONV = [
     (1, 7, 9, 64, 128, 96, 2, False),
     (70, 5, 5, 64, 128, 64, 1, True),        # more tiles than SMs would hold at once is not needed: many images
 ]
+# the eleven MobileNetV2 block shapes again at the cfg3 batch (64 images): one CTA per SM, each working through several
+# output tiles — except the two 10x10-output blocks, whose 128 tiles are fewer than the SMs
+MBCONV += [(64,) + c[1:] for c in MBCONV[:11]]
 
 
 @pytest.mark.parametrize("case", MBCONV)
@@ -293,6 +286,11 @@ def test_mbconv_fused_equals_three_launches(K, case):
     torch.cuda.synchronize()
     info = K.mbconv_last_launch()
     assert got.shape == want.shape
+    if N == 64:
+        ho, wo = got.shape[1:3]
+        tiles = N * -(-ho // info["tile_h"]) * -(-wo // info["tile_w"])
+        assert info["grid"] == min(tiles, K.sm_count()), f"{info}, {tiles} tiles"
+        assert info["grid"] < tiles or ho == 10, f"not persistent: {info}, {tiles} tiles"
     if not torch.equal(got, want):
         diff = (got.float() - want.float()).abs()
         bad = (diff > 0).nonzero()
@@ -329,10 +327,10 @@ def test_grouped_conv_regnet(K, case):
     y = K.conv2d(x.cuda(), K.pack_grouped_weight(w, chunk, c_pad).cuda(), b.cuda(), 3, 3, stride, 1, True,
                  chunk=chunk)
     torch.cuda.synchronize()
-    ref = F.conv2d(x[..., :Cc].float().permute(0, 3, 1, 2).cuda(), w.to(torch.bfloat16).float().cuda(),
-                   b[:Cc].cuda(), stride=stride, padding=1, groups=Cc // gw).relu().permute(0, 2, 3, 1)
-    err = (y[..., :Cc].float() - ref).abs() / ref.abs().clamp(min=1.0)
-    assert y.shape[-1] == c_pad and err.max().item() <= 2e-2, err.max().item()
+    ref, S = conv_ref64(x[..., :Cc].cuda(), w, b[:Cc], stride, 1, groups=Cc // gw, relu=1)
+    assert y.shape[-1] == c_pad
+    worst = assert_bf16_close(y[..., :Cc], ref, S, str(case))
+    print(f"grouped {case}: worst err/tol {worst:.3f}")
     assert (y[..., Cc:] == 0).all()
 
 

@@ -238,3 +238,154 @@ def test_loss_step_host_api_pipelined_batches(P, pinned):
     for o, w in zip(outs, want):
         assert torch.equal(o.clone(), w)
     assert len({tuple(w.tolist()) for w in want}) == 5
+
+
+def test_fused_step_at_cfg4_bench_shape(P):
+    """What bench.py times for cfg4: LossStep(cfg4) at B=16 on the init-style weights (logits clustered around the
+    -4.595 prior bias), the engine's own training-mode logits, the bench targets.  vs extract_targets +
+    MultiBoxLoss.forward_sum per level (depth and num_pos bit-exact, cls_sum 2e-5) and, for one image, vs the numpy
+    oracle (the file's 3e-4 bar)."""
+    import bench
+    import ssds_pytorch_b200 as S
+    from oracle import box_oracle as O
+    from ssds_pytorch_b200 import synth
+    from ssds_pytorch_b200.model import number_box_from_cfg
+    cfg = bench.cfg_dict("cfg4")
+    m = cfg["MODEL"]
+    Bn, C = 16, m["NUM_CLASSES"]
+    nb = number_box_from_cfg(m)
+    assert nb == [9] * 5
+    sd = synth.synthetic_state_dict(m["NETS"], m["FEATURE_LAYER"], nb, C, seed=0, style="init", ssds=m["SSDS"])
+    step = P.LossStep(cfg, sd, use_graph=False)
+    H, W = m["IMAGE_SIZE"]
+    x = torch.randint(0, 256, (Bn, H, W, 3), generator=torch.Generator().manual_seed(1234), dtype=torch.uint8).cuda()
+    tg = synth.synthetic_targets(Bn, seed=4321).cuda()
+    loc, conf = step.model(x)
+    sc, parts = P.fused_loss_step(loc, conf, tg, step.anchors, C, "MultiBoxLoss", None, with_targets=True)
+    torch.cuda.synchronize()
+    assert torch.equal(sc, step.loss_device(x, tg)), "LossStep.loss_device differs from fused_loss_step"
+    crit = S.MultiBoxLoss(3)
+    tot, fg = 0.0, 0.0
+    for li, ((s, anc), c) in enumerate(zip(step.anchors.items(), conf)):
+        hh, ww = c.shape[-2:]
+        A = anc.shape[0]
+        _, _, dep = S.extract_targets(tg, step.anchors, C, s, (hh, ww), [0.5, 0.4], with_cls_target=False)
+        ls, npos = crit.forward_sum(c.view(Bn, A, C, hh, ww), dep)
+        assert torch.equal(parts["depth"][li], dep)
+        assert torch.equal(parts["num_pos"][li], npos)
+        np.testing.assert_allclose(parts["cls_sum"][li].cpu().numpy(), ls.cpu().numpy(), rtol=2e-5, atol=1e-6)
+        tot += ls.double().sum().item()
+        fg += max(npos.sum().item(), 1.0)
+    sc = sc.cpu().numpy()
+    print(f"cfg4 loss step B={Bn}: cls_loss {sc[0]:.6f}, fg {sc[2]:.0f}, logits in "
+          f"[{min(c.min().item() for c in conf):.3f}, {max(c.max().item() for c in conf):.3f}]")
+    assert sc[2] == fg and fg > Bn
+    np.testing.assert_allclose(sc[0], tot / fg, rtol=2e-5)
+    # one image through the numpy oracle
+    i = 5
+    anchors = OrderedDict((s, a.cpu().numpy()) for s, a in step.anchors.items())
+    tgi = tg[i:i + 1].cpu().numpy()
+    for li, ((s, anc), c) in enumerate(zip(anchors.items(), conf)):
+        hh, ww = c.shape[-2:]
+        A = anc.shape[0]
+        cls_t, _, dep = O.extract_targets(tgi, anchors, C, s, (hh, ww), [0.5, 0.4])
+        sums, npos = O.multibox_loss_reduced(c[i:i + 1].cpu().numpy().reshape(1, A, C, hh, ww), cls_t, dep, 3)
+        np.testing.assert_array_equal(parts["depth"][li][i:i + 1].cpu().numpy(), dep)
+        assert parts["num_pos"][li][i].item() == npos[0]
+        np.testing.assert_allclose(parts["cls_sum"][li][i].item(), sums[0], rtol=3e-4)
+
+
+# 16 well-separated values for a negative anchor's largest logit: equal values make exact ties in the hard-negative
+# rank key (max over classes of BCE(x, 0) = softplus(max x)); every other logit of the anchor lies 0.5 - 6 below it,
+# so tied anchors have different CE sums and which of them the cut takes changes the loss
+TIE_LEVELS = np.arange(16, dtype=np.float32) * np.float32(0.25) - np.float32(3.0)
+
+
+def tie_case(seed):
+    """(anchors, levels, targets, conf, depth per level, cls target per level) with the max logits drawn from TIE_LEVELS"""
+    from oracle import box_oracle as O
+    Bn, C = 2, 20
+    levels = [(8, 20), (16, 10), (32, 5)]
+    rng, anchors, tanc, tg, _, loc, A = setup(seed, Bn, C, levels, 6, 160)
+    for b in range(Bn):                    # two boxes per image at the anchor size of each level: positives everywhere
+        for k, (s, _) in enumerate(levels * 2):
+            wh = s * rng.uniform(3.5, 4.6, 2)
+            tg[b, k, :2] = rng.uniform(0, 160 - wh)
+            tg[b, k, 2:4] = wh
+            tg[b, k, 4] = rng.integers(0, C)
+    conf, deps, clss = [], [], []
+    for s, hw in levels:
+        top = rng.choice(TIE_LEVELS, size=(Bn, A, 1, hw, hw))
+        other = top - rng.uniform(0.5, 6.0, (Bn, A, C, hw, hw)).astype(np.float32)
+        arg = rng.integers(0, C, (Bn, A, 1, hw, hw))
+        c = np.where(np.arange(C).reshape(1, 1, C, 1, 1) == arg, top, other).astype(np.float32)
+        conf.append(c.reshape(Bn, A * C, hw, hw))
+        cls_t, _, dep = O.extract_targets(tg, anchors, C, s, (hw, hw), [0.5, 0.4])
+        deps.append(dep)
+        clss.append(cls_t)
+    return anchors, tanc, levels, tg, conf, loc, deps, clss, Bn, A, C
+
+
+def reduced_with_tiebreak(c5, dep, ratio, reverse):
+    """O.multibox_loss_reduced's per-image sums with the rank ties broken by ascending (the criterion's stable sort)
+    or descending index; also the size of the tie group at the cut and how many of it are taken."""
+    from oracle import box_oracle as O
+    ce = O.bce_with_logits(c5, np.zeros_like(c5))          # negatives only carry the key; positives are added below
+    out = []
+    for b in range(c5.shape[0]):
+        key = ce[b].max(axis=1).reshape(-1).copy()
+        d = dep[b].reshape(-1)
+        key[d != 0] = 0
+        idx = np.arange(key.size)
+        order = np.lexsort((-idx if reverse else idx, -key.astype(np.float64)))
+        num_neg = min(ratio * int((d > 0).sum()), key.size - 1)
+        neg = np.zeros(key.size, bool)
+        neg[order[:num_neg]] = True
+        cut = key[order[num_neg - 1]]
+        group = int((key == cut).sum())
+        taken = int((key[order[:num_neg]] == cut).sum())
+        out.append((neg, cut, group, taken, key[order[num_neg]]))
+    return out
+
+
+def test_hard_negative_selection_breaks_ties_by_index(P):
+    """The hard-negative cut falls INSIDE a group of exactly equal rank keys in every (image, level): which of the tied
+    anchors are taken (the lower indices, criterion.py's stable descending sort) decides the loss.
+      * MultiBoxLoss.forward's mask (out != 0) == O.multibox_loss's mask, exactly;
+      * the fused step's per-pair cls_sum and MultiBoxLoss.forward_sum == O.multibox_loss_reduced within 5e-6: the
+        fast softplus has 2.3e-7 relative error per term and fp32 partial sums of a few thousand positive terms
+        add < 1e-6, so 5e-6 is ample for a correct kernel;
+      * the oracle with the REVERSED tie-break (higher index first) is at least 10x that tolerance away in every
+        pair, so a kernel that cuts the tie group at the wrong end cannot pass."""
+    import ssds_pytorch_b200 as S
+    from oracle import box_oracle as O
+    rtol = 5e-6
+    anchors, tanc, levels, tg, conf, loc, deps, clss, Bn, A, C = tie_case(1)
+    sc, parts = P.fused_loss_step([torch.from_numpy(x).cuda() for x in loc], [torch.from_numpy(x).cuda() for x in conf],
+                                  torch.from_numpy(tg).cuda(), tanc, C, "MultiBoxLoss", None, with_targets=True)
+    crit = S.MultiBoxLoss(3)
+    for li, ((s, hw), c, dep, cls_t) in enumerate(zip(levels, conf, deps, clss)):
+        c5 = c.reshape(Bn, A, C, hw, hw)
+        want, npos = O.multibox_loss_reduced(c5, cls_t, dep, 3)
+        ce = O.bce_with_logits(c5, cls_t)
+        cuts = reduced_with_tiebreak(c5, dep, 3, reverse=False)
+        cuts_r = reduced_with_tiebreak(c5, dep, 3, reverse=True)
+        for b in range(Bn):
+            neg, cut, group, taken, nxt = cuts[b]
+            assert nxt == cut and 0 < taken < group, f"level {li} image {b}: the cut is not inside a tie group"
+            m_r = (dep[b] > 0) | cuts_r[b][0].reshape(dep[b].shape)
+            sum_r = (ce[b] * m_r * (dep[b] >= 0)).astype(np.float64).sum()
+            margin = abs(sum_r - want[b]) / abs(want[b])
+            print(f"level {li} image {b}: num_pos {npos[b]}, tie group of {group} at key {cut:.6f}, {taken} taken; "
+                  f"reversed tie-break moves the sum by {margin:.2e} (tolerance {rtol:.0e})")
+            assert margin >= 10 * rtol
+        # the unreduced drop-in: same mask
+        mask_o = O.multibox_loss(c5, cls_t, dep, 3) != 0
+        out = crit(torch.from_numpy(c5).cuda(), torch.from_numpy(cls_t).cuda(), torch.from_numpy(dep).cuda())
+        mask_g = (out != 0).cpu().numpy()
+        assert (mask_g == mask_o).all(), f"level {li}: {int((mask_g != mask_o).sum())} mask elements differ"
+        ls, npos_g = crit.forward_sum(torch.from_numpy(c5).cuda(), torch.from_numpy(dep).cuda())
+        np.testing.assert_array_equal(npos_g.cpu().numpy(), npos.astype(np.float32))
+        np.testing.assert_array_equal(parts["depth"][li].cpu().numpy(), dep)
+        np.testing.assert_allclose(ls.cpu().numpy(), want, rtol=rtol)
+        np.testing.assert_allclose(parts["cls_sum"][li].cpu().numpy(), want, rtol=rtol)
